@@ -1,2 +1,2 @@
-"""Reference arm of bench.py: the UNMODIFIED reference installed under baseline/_ref/ (git-ignored,
-travels to the GPU box with the snapshot).  See install_ref.sh / ref_loader.py."""
+"""Reference arm of bench.py and the drop-in tests: the UNMODIFIED reference, installed under oracle/_ref/
+(not under version control) by build().  See oracle/ref_install.py / ref_loader.py."""

@@ -242,13 +242,16 @@ def run_cuda(args):
     def train_resident(i):
         tr.train_batch_device(devin[i][0])   # fused step; at world > 1 data-parallel inside the Trainer
 
+    # device tensor holding the loss of the latest resident step (every launch mode points it at its own buffer)
+    last = {"loss": None}
+
     def resident_step(i):
         if graph_step is not None:
             return graph_step(i)
         # multi-GPU "ids" mode: the 24 KB id all-gather is started first and hides behind the evaluation batch
         ex = tr.exchange_batch_async(devin[i][0])
         eval_resident(i)
-        tr.train_batch_device(devin[i][0], exchanged=ex)
+        last["loss"] = tr.train_batch_device(devin[i][0], exchanged=ex)
 
     # Single GPU: the resident step is ~12 short kernels, so launch gaps are a visible share of it.  It is
     # captured ONCE as a CUDA graph reading from fixed device buffers; a timed step is then the D2D copies of
@@ -313,6 +316,7 @@ def run_cuda(args):
                 _lib.train_pairwise_hinge_sgd(desc, scratch, *s_ids, w["margin"], lr, loss_buf)
 
             g, kernels_per_replay = capture(lambda: body(w["lr"]), lambda: body(0.0))
+            last["loss"] = loss_buf
             # the two halves as graphs of their own, for the separately reported train / eval rates
             g_eval, _ = capture(body_eval, body_eval)
             g_train, _ = capture(lambda: _lib.train_pairwise_hinge_sgd(desc, scratch, *s_ids, w["margin"], w["lr"], loss_buf),
@@ -341,7 +345,8 @@ def run_cuda(args):
                 return [gl[k] for k in range(6)]
 
             def body_train():
-                tr.train_batch_device(s_ids, exchanged=glob_ids)
+                # the call made during capture leaves the graph's own loss buffer here
+                last["loss"] = tr.train_batch_device(s_ids, exchanged=glob_ids)
 
             def warm_train():
                 lr0 = tr.config.learning_rate
@@ -442,7 +447,9 @@ def run_cuda(args):
 
     # sustained run (~1.5 s of back-to-back steps) so that nvidia-smi samples clocks UNDER LOAD.  The number of
     # passes is fixed from one timed pass and agreed across ranks (MAX): a time-based loop would let the ranks
-    # run different numbers of steps, and the steps contain collectives.
+    # run different numbers of steps, and the steps contain collectives.  Its training updates are undone
+    # afterwards, so that the timed steps start from tables that depend on the arguments only, not on the clock.
+    tables0 = [t_.detach().clone() for t_ in tr.model.kge_tables()]
     torch.cuda.synchronize()
     t_p0 = time.perf_counter()
     for i in range(args.warmup, total):
@@ -460,6 +467,10 @@ def run_cuda(args):
             resident_step(i)
         torch.cuda.synchronize()
     ms_sustained = (time.perf_counter() - t_s0) * 1e3 / (n_pass * args.steps)
+    with torch.no_grad():
+        for t_, t0_ in zip(tr.model.kge_tables(), tables0):
+            t_.copy_(t0_)
+    del tables0
     barrier()
     import gc
     gc.collect()
@@ -467,6 +478,13 @@ def run_cuda(args):
     launches0 = _lib.launch_count()
     ms_res = max_over_ranks(timed(resident_step, args.warmup, args.steps, True))
     launches = _lib.launch_count() - launches0
+    # what the last timed step returned (this rank's rank counts, the loss) and left behind (the trained tables)
+    counts_last = counts.clone()
+    dump = None
+    if args.dump_outputs and rank == 0:
+        names = ("ent_embeddings", "rel_embeddings")
+        dump = {"loss": last["loss"].detach().reshape(1).float().cpu().numpy()}
+        dump.update({n: t_.detach().float().cpu().numpy() for n, t_ in zip(names, tr.model.kge_tables())})
     if graph_step is not None:
         launches = kernels_per_replay * args.steps   # replays re-execute the captured kernels
     ms_train = max_over_ranks(timed(train_resident, args.warmup, args.steps, True))
@@ -482,9 +500,11 @@ def run_cuda(args):
     ms_warm = max_over_ranks(a.elapsed_time(b))
     ms_e2e = max_over_ranks(timed(e2e_step, args.warmup, args.steps, False)) if not args.lite else float("nan")
     gc.enable()
-    # multi-GPU: the ranks of all shards are gathered ONCE, after the timing (one all-gather of Q x 4 int32)
-    if world > 1:
-        sharding.gather_query_shards(counts.clone(), world * w["Q"])
+    # multi-GPU: the ranks of all shards (those of the last timed step) are gathered ONCE, after the timing
+    # (one all-gather of Q x 4 int32)
+    all_counts = sharding.gather_query_shards(counts_last, world * w["Q"]) if world > 1 else counts_last
+    if dump is not None:
+        dump["rank_counts"] = all_counts.cpu().numpy().astype(np.float64)
 
     # ---- dominant kernel of the step: the tensor-core sweep, timed alone with CUDA events recorded around
     # the kernel launch itself on its own stream (C-ABI profiling hook), L2 flushed before every launch
@@ -556,6 +576,10 @@ def run_cuda(args):
         "rooflines_extra": extra,
         "cpu_baseline": cpu,
     }
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     return line
 
 
@@ -574,7 +598,7 @@ def usable_cores():
 
 
 class RefArm:
-    """The UNMODIFIED reference (baseline/_ref, pip-installed from /root/reference) on the host cores, driven
+    """The UNMODIFIED reference (oracle/_ref, installed by build(): oracle/ref_install.py) on the host cores, driven
     through its own code: pykg2vec.models.pairwise.TransE, Trainer.train_step_pairwise + backward +
     optimizer.step (pykg2vec/utils/trainer.py:147-157,288-300) and Evaluator.test
     (pykg2vec/utils/evaluator.py:309-334: two forwards over all N entities, topk(N), D2H, the Python rank walk
@@ -607,7 +631,7 @@ class RefArm:
         self.batches = make_batches(self.kg, 64, 0)
         self.test = self.kg.read_cache_data("triplets_test")
         self.cursor = 0
-        self.desc = "torch %s CPU, pykg2vec 0.0.52 from baseline/_ref" % torch.__version__
+        self.desc = "torch %s CPU, pykg2vec 0.0.52 from oracle/_ref" % torch.__version__
 
     def train_steps(self, n):
         torch = self.torch
@@ -635,7 +659,7 @@ class RefArm:
 
 
 class PortArm:
-    """Fallback when baseline/_ref is absent: the torch port of the same op chain (oracle/ref_port.py)."""
+    """Fallback when oracle/_ref is absent: the torch port of the same op chain (oracle/ref_port.py)."""
     kind = "port"
 
     def __init__(self):
@@ -688,7 +712,7 @@ def make_arm():
         try:
             return RefArm()
         except Exception as e:   # noqa: BLE001 — fall back to the port, say why
-            sys.stderr.write("reference arm: baseline/_ref unusable (%r), using the port\n" % (e,))
+            sys.stderr.write("reference arm: oracle/_ref unusable (%r), using the port\n" % (e,))
     return PortArm()
 
 
@@ -778,7 +802,14 @@ def main():
                     help="launch the resident step kernel by kernel instead of replaying it as one CUDA graph (N = 1)")
     ap.add_argument("--lite", action="store_true",
                     help="profiling aid: only the HBM-resident leg (no e2e / CPU baseline / self-check); never a bench value")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy: rank_counts "
+                         "((GPUs x Q) x 4, the query shards of all ranks in rank order: tail raw, tail filtered, head raw, "
+                         "head filtered; float64), rank 0's loss (float32) and the "
+                         "trained ent_embeddings / rel_embeddings (float32); the same arguments give the same inputs")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "cuda" or args.config != 2):
+        ap.error("--dump-outputs writes the outputs of the CUDA path's headline step (--impl cuda --config 2)")
     if args.config != 2:
         import bench_sharded
         return bench_sharded.main(["--queries", "512" if args.config == 5 else "4096"], only=args.config)

@@ -44,6 +44,15 @@ def install_reference():
     mpl.pyplot = plt
     sys.modules.update({"hyperopt": ho, "hyperopt.pyll": pyll, "hyperopt.pyll.base": base,
                         "seaborn": sb, "matplotlib": mpl, "matplotlib.pyplot": plt})
+    # utils/visualization.py:11-14, reached through pykg2vec.utils.trainer: stubbed when not installed
+    import importlib.util
+    if importlib.util.find_spec("networkx") is None:
+        sys.modules["networkx"] = types.ModuleType("networkx")
+    if importlib.util.find_spec("sklearn") is None:
+        sk, manifold = types.ModuleType("sklearn"), types.ModuleType("sklearn.manifold")
+        manifold.TSNE = None
+        sk.manifold = manifold
+        sys.modules.update({"sklearn": sk, "sklearn.manifold": manifold})
 
 
 install_reference()

@@ -8,7 +8,7 @@ reference classes — the product has no CPU path by design (a CPU fallback woul
 test_config1_cli_flow_reference_cpu runs exactly that flow here on the UMLS-shaped synthetic dataset, and
 the -m gpu tests run the same flow through the B200 classes with `-device cuda`.
 
-Needs baseline/_ref (the unmodified reference, installed by baseline/install_ref.sh; travels to the GPU box)."""
+Needs oracle/_ref (the unmodified reference, installed there by build() from a checkout of it: oracle/ref_install.py)."""
 import os
 import sys
 
@@ -19,7 +19,7 @@ import torch
 import dropin_util as du
 from baseline import ref_loader
 
-needs_ref = pytest.mark.skipif(not ref_loader.available(), reason="baseline/_ref not installed (baseline/install_ref.sh)")
+needs_ref = pytest.mark.skipif(not ref_loader.available(), reason="oracle/_ref not installed (build() installs it from a checkout of the reference)")
 CFG1 = ["-mn", "TransE", "-l", "2", "-ts", "1", "-tn", "50", "-npg", "1"]   # defaults otherwise: d=50, B=128, adam, L1, margin 0.8
 
 
@@ -104,5 +104,30 @@ def test_pretrained_checkpoint_loads_through_trainer_load_model(tmp_path, monkey
     with torch.no_grad():
         want = ref(h, r, t).numpy()
         got = m(h.cuda(), r.cuda(), t.cuda()).cpu().numpy()
+    err = np.abs(got - want) / np.maximum(np.abs(want), 1e-2 * np.abs(want).max())
+    assert err.max() < 1e-4, err.max()
+
+
+@pytest.mark.gpu
+def test_pretrained_checkpoint_scores_match_reference_golden():
+    """The same checkpoint without the reference installed (tests/golden/make_golden_dropin.py): the B200
+    TransE built from the constructor arguments the reference's Trainer.load_model passed takes a state_dict
+    in the checkpoint's layout and shape (the rows 1,024 seeded triples touch, the rest zero) and scores
+    those triples as the reference class did."""
+    import pykg2vec_b200
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pretrained_transe_fb15k_checkpoint.npz"))
+    n_ent, n_rel, d = int(g["tot_entity"]), int(g["tot_relation"]), int(g["hidden_size"])
+    m = pykg2vec_b200.import_model(str(g["model_name"]))(tot_entity=n_ent, tot_relation=n_rel, hidden_size=d,
+                                                         l1_flag=bool(g["l1_flag"]))
+    assert type(m).__module__ == "pykg2vec_b200.pairwise"
+    ent, rel = torch.zeros(n_ent, d), torch.zeros(n_rel, d)
+    ent[torch.from_numpy(g["ent_ids"])] = torch.from_numpy(g["ent_rows"])
+    rel[torch.from_numpy(g["rel_ids"])] = torch.from_numpy(g["rel_rows"])
+    m.load_state_dict({"ent_embeddings.weight": ent, "rel_embeddings.weight": rel})
+    m = m.cuda().eval()
+    h, r, t = (torch.from_numpy(g[k]).cuda() for k in ("h", "r", "t"))
+    with torch.no_grad():
+        got = m(h, r, t).cpu().numpy()
+    want = g["scores"]
     err = np.abs(got - want) / np.maximum(np.abs(want), 1e-2 * np.abs(want).max())
     assert err.max() < 1e-4, err.max()

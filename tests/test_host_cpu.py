@@ -27,7 +27,13 @@ def test_library_builds_loads_and_exports_every_declared_symbol():
     L = _lib.lib()
     assert L.kge_abi_version() == _lib.ABI_VERSION
     assert b"sm_100a" in L.kge_version()
-    assert L.kge_launch_count() == 0  # loading the library touches no CUDA state
+    # loading the library touches no CUDA state; checked in a fresh interpreter, because GPU tests run
+    # earlier in this process launch kernels through the same loaded library
+    import subprocess
+    import sys
+    code = "import sys; sys.path.insert(0, sys.argv[1]); from pykg2vec_b200 import _lib; print(_lib.lib().kge_launch_count())"
+    res = subprocess.run([sys.executable, "-c", code, ROOT], capture_output=True, text=True, check=True)
+    assert int(res.stdout.split()[-1]) == 0
 
 
 def test_sass_shows_the_blackwell_instructions_the_design_claims():
